@@ -24,6 +24,8 @@ torch.distributed.run, one rank per GPU.  Rank 0 prints ONE JSON line.
   cpu_baseline   the CPU oracle (threaded C++ restatement of the halo2 prover; the Rust reference cannot be built in
             this image) timed on this box's host cores on a bounded sample (1 Compliance + 1 VP proof -> ptx/s).
   --impl reference   times that CPU arm alone, same metric / config (see DESIGN.md "Reference arm").
+  --dump-outputs DIR   writes the proofs of the last timed step (rank 0) as DIR/compliance_proofs.npy and DIR/vp_proofs.npy,
+            one row of proof bytes per proof in float32, so that two builds can be compared output for output.
 Synthetic data: Taiga-shaped circuits with satisfying witnesses (taiga_b200/circuits_taiga.py), a distinct witness per
 proof; a sample of the proofs of the last timed step is checked with the oracle's verifier restatement and ALL of them
 with the device verifier, outside the timed region.
@@ -324,6 +326,22 @@ def emit(line):
     _REAL_STDOUT.flush()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, records):
+    """records: {name: list of equal-length proof byte strings}.  Writes out_dir/<name>.npy, float32 [proofs, bytes] (exact for
+    bytes).  Above DUMP_LIMIT_BYTES in all, every array keeps the same share of its rows, a sample fixed by seed 0."""
+    arrays = {k: np.frombuffer(b"".join(v), np.uint8).reshape(len(v), -1) for k, v in records.items()}
+    total = sum(4 * a.size for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = len(a) * DUMP_LIMIT_BYTES // total
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def ncu_traffic():
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernels, from the committed ncu capture
     (written by profiles/extract_ncu_traffic.py from the raw page of the .ncu-rep; not a constant in this file)."""
@@ -359,7 +377,12 @@ def main():
     ap.add_argument("--no-synth-pipeline", action="store_true")
     ap.add_argument("--all-probes", action="store_true", help="multi-GPU runs skip the secondary probes (single-ptx latency, overlapped synthesis) unless this is given")
     ap.add_argument("--serial", action="store_true", help="one stream, no threads (for ncu launch lists; not a benchmark configuration)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proofs of the last timed step as DIR/<name>.npy (float32 bytes)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's proofs; the reference arm makes none")
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -552,6 +575,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"compliance_proofs": last[0], "vp_proofs": last[1]})
 
     # acceptance (outside the timed region): a sample of the last e2e step under the oracle's verifier restatement (35 ms/proof of
     # CPU each), ALL of its proofs under the library's batched device verifier (tb_verify_batch, SURVEY 8 (f)-3)
