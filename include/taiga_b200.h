@@ -144,6 +144,18 @@ tb_status tb_prove_batch(tb_ctx* ctx, const tb_pk* pk, uint32_t n_proofs, const 
 tb_status tb_verify_batch(tb_ctx* ctx, const tb_pk* pk, uint32_t n_proofs, const uint8_t* instance, const uint32_t* instance_len,
                           const uint8_t* proofs, size_t proof_stride, size_t proof_len, uint8_t* ok_out);
 
+/* Constraint check of n_proofs witnesses of one circuit (halo2 dev::MockProver::verify; the reference's
+ * verify_transparently, resource_logic_circuit.rs:597-606).  advice / instance / instance_len as in tb_prove_batch
+ * (host, pinned-host or device memory; instance_len on the host).  Advice cells in the last blinding_factors+1 rows are
+ * poison whatever they hold.  Per proof, tb_pk_check_slots(pk) = 2C + L + P slots:
+ *   [0, C) constraint j unsatisfied | [C, 2C) constraint j poisoned | [2C, 2C+L) lookup l | [2C+L, 2C+L+P) copy, permutation column p
+ * fail_rows[i*S + s] = number of failing rows, first_row[i*S + s] = lowest failing row (0xFFFFFFFF if none).
+ * Proof i satisfies the circuit iff all its fail_rows are 0.  1 <= n_proofs <= 4096.  Errors: TB_ERR_INVALID for
+ * malformed arguments, instance_len > usable rows (InstanceTooLarge) and a sigma value that names no cell. */
+size_t    tb_pk_check_slots(const tb_pk* pk);
+tb_status tb_check_batch(tb_ctx* ctx, const tb_pk* pk, uint32_t n_proofs, const uint8_t* advice, const uint8_t* instance,
+                         const uint32_t* instance_len, uint32_t* fail_rows, uint32_t* first_row);
+
 #ifdef __cplusplus
 }
 #endif

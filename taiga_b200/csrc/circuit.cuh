@@ -19,6 +19,21 @@ struct WsBlock { void* p = nullptr; size_t bytes = 0; };
 // with the SAME context and batch size while a call is in flight is refused (TB_ERR_INVALID) instead of corrupting it.
 struct ProveWs { std::vector<WsBlock> blocks; std::vector<void*> tables; std::vector<std::vector<uint8_t>> table_bytes; std::atomic<int> busy{0}; };
 
+// What tb_check_batch needs of a key beyond the prover's tables (check.cu), built on the first check and read-only afterwards.
+struct CheckKey {
+  QProgram gates, lk_in, lk_tab;   // Q_CK_TEST per constraint; Q_CK_STORE per lookup input / table expression
+  int E = 0;                       // lookup expressions over all lookups
+  int2* d_lk = nullptr;            // per lookup: (first expression slot, expressions)
+  uint32_t* perm_map = nullptr;    // [P][n]: the cell sigma sends (column p, row r) to, packed p' << 24 | r'
+  // tables that read only fixed columns and constants, evaluated and sorted once: [L][n] row order, [E][n] values, [L][n] poison
+  bool tables_fixed = false;
+  uint32_t* tab_idx = nullptr; Fp* tab_vals = nullptr; uint8_t* tab_pois = nullptr;
+  ~CheckKey() {
+    for (void* p : {(void*)d_lk, (void*)perm_map, (void*)tab_idx, (void*)tab_vals, (void*)tab_pois, (void*)gates.dev, (void*)lk_in.dev, (void*)lk_tab.dev})
+      if (p) cudaFree(p);
+  }
+};
+
 struct Circuit {
   Ctx* ctx; const Srs* srs;
   // deep copy of the description
@@ -46,9 +61,10 @@ struct Circuit {
   std::vector<PolyId> uniq; std::vector<int> uniq_set; std::vector<std::vector<int>> point_sets;
   uint32_t proof_len;
   // persistent per-batch-size workspace and cached small tables (see prove_batch)
-  mutable std::mutex mu;                                                   // guards the two caches below
+  mutable std::mutex mu;                                                   // guards the three caches below
   mutable std::map<std::pair<const Ctx*, int>, std::unique_ptr<ProveWs>> ws;
   mutable std::vector<Aff<Fq>> vk_fixed, vk_sigma;   // verifying-key commitments (Montgomery, host), filled on first verification
+  mutable std::unique_ptr<CheckKey> check;           // constraint-check tables, filled on the first tb_check_batch
   ProveWs& workspace(const Ctx* c, int B) const {
     std::lock_guard<std::mutex> lk(mu);
     auto& slot = ws[std::make_pair(c, B)];

@@ -12,7 +12,9 @@ void lookup_arrange(Ctx* c, const Fp* sortedA, const Fp* sortedT, Fp* scratch, F
 // ---------------------------------------------------------------- quotient.cu
 // Row-parallel expression interpreter (SURVEY.md App. E.6).  Temporaries live in a shared-memory register file laid
 // out [reg][thread] as two 16-byte halves; leaves (column queries, constants) are read straight from global memory.
-enum QOp { Q_MOV = 0, Q_NEG, Q_ADD, Q_SUB, Q_MUL, Q_FOLD_Y, Q_LK_BEGIN, Q_FOLD_A, Q_FOLD_S, Q_LK_STORE, Q_GBEGIN, Q_GFOLD, Q_GEND };
+// Q_CK_TEST / Q_CK_STORE end the constraint-check programs (check.cu): test the operand as constraint `b`, or store it as lookup
+// expression `b` of lookup `pad`.
+enum QOp { Q_MOV = 0, Q_NEG, Q_ADD, Q_SUB, Q_MUL, Q_FOLD_Y, Q_LK_BEGIN, Q_FOLD_A, Q_FOLD_S, Q_LK_STORE, Q_GBEGIN, Q_GFOLD, Q_GEND, Q_CK_TEST, Q_CK_STORE };
 enum QKind { K_REG = 0, K_ADV, K_FIX, K_INST, K_CONST };
 struct alignas(16) QInstr { uint32_t w0; uint32_t a, b, pad; };  // w0 = op | dst << 8 | akind << 16 | bkind << 24 (one 128-bit load)
 inline QInstr q_make(int op, int dst, int ak, uint32_t a, int bk, uint32_t b) { QInstr i; i.w0 = op | (dst << 8) | (ak << 16) | (bk << 24); i.a = a; i.b = b; i.pad = 0; return i; }
@@ -33,6 +35,10 @@ void q_compile_gates_split(const tb_cs_desc* cs, const std::vector<uint32_t>& su
 std::vector<int> q_constraint_degrees(const tb_cs_desc* cs);
 struct QPartList { const QInstr* prog[Q_MAX_PARTS]; int ninstr[Q_MAX_PARTS]; int nparts; long long part_stride; };
 void q_compile_lookups(const tb_cs_desc* cs, QProgram* out);
+// constraint-check programs: every constraint root followed by Q_CK_TEST j; or every lookup input (tables = false) / table
+// (tables = true) expression followed by Q_CK_STORE, expressions numbered lookup-major across all lookups
+void q_compile_check_gates(const tb_cs_desc* cs, QProgram* out);
+void q_compile_check_lookups(const tb_cs_desc* cs, bool tables, QProgram* out);
 
 struct QData {
   const Fp* adv; long long adv_pstride;     // [B][num_advice][n]

@@ -225,6 +225,33 @@ void q_compile_lookups(const tb_cs_desc* cs, QProgram* out) {
   finish_program(c, out);
 }
 
+void q_compile_check_gates(const tb_cs_desc* cs, QProgram* out) {
+  Compiler c(cs);
+  std::vector<char> seen(cs->num_nodes, 0);
+  for (uint32_t j = 0; j < cs->num_constraints; ++j) c.count(cs->constraint_roots[j], seen);
+  for (uint32_t j = 0; j < cs->num_constraints; ++j) {
+    Compiler::Opnd o = c.emit(cs->constraint_roots[j]);
+    c.code.push_back(q_make(Q_CK_TEST, 0, o.kind, o.v, K_CONST, j)); c.release(o);
+  }
+  finish_program(c, out);
+}
+
+void q_compile_check_lookups(const tb_cs_desc* cs, bool tables, QProgram* out) {
+  Compiler c(cs);
+  std::vector<char> seen(cs->num_nodes, 0);
+  auto root = [&](uint32_t l, uint32_t e) { return tables ? cs->lookups[l].table_roots[e] : cs->lookups[l].input_roots[e]; };
+  for (uint32_t l = 0; l < cs->num_lookups; ++l)
+    for (uint32_t e = 0; e < cs->lookups[l].num_exprs; ++e) c.count(root(l, e), seen);
+  uint32_t slot = 0;
+  for (uint32_t l = 0; l < cs->num_lookups; ++l)
+    for (uint32_t e = 0; e < cs->lookups[l].num_exprs; ++e) {
+      Compiler::Opnd o = c.emit(root(l, e));
+      QInstr in = q_make(Q_CK_STORE, 0, o.kind, o.v, K_CONST, slot++); in.pad = l;
+      c.code.push_back(in); c.release(o);
+    }
+  finish_program(c, out);
+}
+
 // ---------------------------------------------------------------- interpreter kernel
 // One thread per (row, constraint part).  ALL values, including the running folds, live in the shared-memory register file
 // [nregs + 2][T] x 32 B (slot nregs = the y / theta fold accumulator, slot nregs + 1 = the group / table fold): the loop carries

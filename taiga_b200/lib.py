@@ -57,7 +57,44 @@ _SIGS = {
     "tb_pk_commitments": (_i, [_vp, _vp, _vp, _vp]),
     "tb_prove_batch": (_i, [_vp, _vp, _u32, _vp, _vp, _vp, _vp, _u32, _vp, _sz]),
     "tb_verify_batch": (_i, [_vp, _vp, _u32, _vp, _vp, _vp, _sz, _sz, _vp]),
+    "tb_pk_check_slots": (_sz, [_vp]),
+    "tb_check_batch": (_i, [_vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
 }
+
+
+class CheckReport:
+    """Constraint-check result of one witness (halo2 `MockProver::verify`).  `fail_rows` / `first_row` are the witness's
+    tb_check_batch slots; `failures` lists (kind, index, first_row, rows) with kind "gate" (constraint unsatisfied),
+    "poisoned" (constraint reads a blinding-row advice cell), "lookup" or "copy" (permutation column index)."""
+
+    def __init__(self, fail_rows, first_row, num_constraints, num_lookups):
+        self.fail_rows, self.first_row = fail_rows, first_row
+        C, L = num_constraints, num_lookups
+        self.failures = []
+        for s in np.flatnonzero(fail_rows):
+            s = int(s)
+            kind, idx = ("gate", s) if s < C else ("poisoned", s - C) if s < 2 * C else ("lookup", s - 2 * C) if s < 2 * C + L else ("copy", s - 2 * C - L)
+            self.failures.append((kind, idx, int(first_row[s]), int(fail_rows[s])))
+        self.ok = not self.failures
+
+    def describe(self, keydata):
+        """One line per failure, named as MockProver names it: gate name and polynomial index, lookup index, permutation column."""
+        cs = keydata.cs
+        polys = [(name, i) for name, ps in cs.gates for i in range(len(ps))]
+        out = []
+        for kind, idx, row, rows in self.failures:
+            if kind in ("gate", "poisoned"):
+                name, i = polys[idx]
+                what = "constraint %d of gate %r %s" % (i, name, "not satisfied" if kind == "gate" else "reads a poisoned cell")
+            elif kind == "lookup":
+                what = "lookup %d input not in its table" % idx
+            else:
+                what = "copy constraint on column %r broken" % cs.perm_columns[idx]
+            out.append("%s: first at row %d (%d rows)" % (what, row, rows))
+        return out
+
+    def __repr__(self):
+        return "CheckReport(ok=%s, failures=%r)" % (self.ok, self.failures)
 
 
 def exported_symbols():
@@ -277,6 +314,29 @@ class ProvingKey:
         ok = np.zeros(B, np.uint8)
         ctx._check(ctx._lib.tb_verify_batch(ctx._h, self._h, B, _ptr(inst), _ptr(lens), _ptr(buf), plen, plen, _ptr(ok)))
         return [bool(v) for v in ok]
+
+    def check_batch(self, advice, instance, instance_len, ctx=None):
+        """MockProver::verify for a batch: advice uint8 [B, num_advice, n, 32]; instance uint8 [B, sum(instance_len), 32].
+        Returns one CheckReport per witness."""
+        adv = _u8(advice)
+        kd = self.keydata
+        per = kd.cs.num_advice * kd.n * 32
+        assert adv.size % per == 0
+        return self.check_batch_raw(adv, adv.size // per, instance, instance_len, ctx=ctx)
+
+    def check_batch_raw(self, advice, B, instance, instance_len, ctx=None):
+        """Same, with `advice` given as anything exposing its address (numpy array, pinned-host or DEVICE torch tensor)."""
+        ctx = ctx or self.ctx
+        inst = _u8(instance)
+        lens = np.ascontiguousarray(instance_len, dtype=np.uint32)
+        assert inst.size >= B * int(lens.sum()) * 32
+        S = int(ctx._lib.tb_pk_check_slots(self._h))
+        fail = np.zeros((B, max(1, S)), np.uint32)
+        first = np.zeros((B, max(1, S)), np.uint32)
+        ctx._check(ctx._lib.tb_check_batch(ctx._h, self._h, B, _ptr(advice), _ptr(inst), _ptr(lens), _ptr(fail), _ptr(first)))
+        cs = self.keydata.cs
+        C = sum(len(ps) for _, ps in cs.gates)
+        return [CheckReport(fail[b, :S], first[b, :S], C, len(cs.lookups)) for b in range(B)]
 
     def close(self):
         if getattr(self, "_h", None):

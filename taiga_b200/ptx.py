@@ -9,6 +9,7 @@
       2 x ComplianceVerifyingInfo::create + 4 x get_verifying_info, sequential
                                                                          ProverService.build_ptx_batch: all 2P Compliance proofs
                                                                          in one batched call, all 4P VP proofs in another
+  verify_transparently  resource_logic_circuit.rs:597-606      ProverService.check_ptx_batch (MockProver::verify on the GPU)
 
 The circuits are the Taiga-shaped ones of circuits_taiga.py (the real ones need the Rust `synthesize`).  Witness
 synthesis happens on the host before the call, exactly as `Circuit::synthesize` does in the reference; it is not part
@@ -116,6 +117,12 @@ class ProverService:
         for (kind, lo) in sorted(results):
             out[kind] += results[(kind, lo)]
         return out["c"], out["v"]
+
+    def check_ptx_batch(self, wit):
+        """The batched counterpart of `verify_transparently` (resource_logic_circuit.rs:597-606): MockProver::verify of every
+        witness of a synthesized batch.  Returns (compliance CheckReports, vp CheckReports)."""
+        return (self.pk_c.check_batch(wit["c_adv"], wit["c_inst"], wit["c_len"]),
+                self.pk_v.check_batch(wit["v_adv"], wit["v_inst"], wit["v_len"]))
 
     @property
     def launch_count(self):
